@@ -21,6 +21,8 @@ Product arm:
   match    MatchSiftData 2000 x 2000 and 10000 x 10000 (BASELINE config #3), exact and tensor-core paths
   allpairs (N > 1) BASELINE config #5: per-GPU ExtractSift + ONE NCCL all-gather + all-pairs match
   cpu_baseline (N = 1) the oracle port on the host cores + OpenCV SIFT
+  --dump-outputs DIR  writes the keypoints of the last timed step as .npy files (dump_outputs), so that two builds can be
+           compared output for output on the same seeded inputs
 Reference arm (--impl reference): the unmodified reference library (oracle/_ref/libcudasift_ref.so) through its own
 C++ API in a process that never loads libcudasift_b200.so: same images, same config, same statistics.
 One JSON line on stdout (rank 0).
@@ -284,6 +286,8 @@ def run_product(args):
     n_images = args.steps * B * R * world
     value = n_images / (dev_ms / 1e3)
     pts_per_image = float(np.mean(counts))            # all B images of the last step
+    if args.dump_outputs and rank == 0:               # outside the timed region, before anything reuses the record slots
+        dump_outputs(args.dump_outputs, [exs[s].device_points_at(i, counts[s * b + i]) for s in range(S) for i in range(b)])
 
     # --- timed region 2: end to end through the C ABI with host (pinned) buffers ---
     hptrs = []
@@ -349,6 +353,31 @@ def run_product(args):
     if dist is not None:
         dist.barrier()
         dist.destroy_process_group()
+
+
+DUMP_FIELDS = ("xpos", "ypos", "scale", "sharpness", "edgeness", "orientation", "subsampling")
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, per_image):
+    """What ExtractSift hands its caller for each image of the last timed step, as float arrays:
+    counts.npy (float64, keypoints per image), keypoints.npy (float32, one row of DUMP_FIELDS per keypoint) and
+    descriptors.npy (float32, 128 per keypoint); images in order, each image's keypoints in canonical order (the device
+    appends them in no fixed order).  The match fields of the records are not written: extraction leaves them unset.
+    Above DUMP_MAX_BYTES in all, a fixed seeded sample of keypoint rows is written, and rows.npy (float64) names them."""
+    os.makedirs(out_dir, exist_ok=True)
+    recs = np.concatenate([p[np.lexsort((p["orientation"], p["scale"], p["xpos"], p["ypos"], p["subsampling"]))]
+                           for p in per_image])
+    out = {"counts": np.array([len(p) for p in per_image], np.float64),
+           "keypoints": np.stack([recs[f] for f in DUMP_FIELDS], axis=1).astype(np.float32),
+           "descriptors": np.ascontiguousarray(recs["data"], np.float32)}
+    row_bytes = 4 * (len(DUMP_FIELDS) + 128)
+    room = DUMP_MAX_BYTES - out["counts"].nbytes - 4 * 128           # 128: the header of each .npy file
+    if len(recs) * row_bytes > room:
+        rows = np.sort(np.random.default_rng(0).choice(len(recs), room // (row_bytes + 8), replace=False))
+        out.update(keypoints=out["keypoints"][rows], descriptors=out["descriptors"][rows], rows=rows.astype(np.float64))
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def bench_dropin(cs, imgs, pitch, n=48):
@@ -739,7 +768,10 @@ def main():
     ap.add_argument("--streams", type=int, default=2, help="batch extractors in flight (batch / streams images each)")
     ap.add_argument("--distinct", type=int, default=8, help="distinct synthetic images per rank")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the keypoints of the last timed step to DIR/*.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the product computed; the reference arm has no dump")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -58,3 +58,24 @@ def compare_sets(a, b, **kw):
         out["desc_bad"] = int((dd[finite].max(axis=1) > 1e-3).sum())
         out["sharp_rel"] = float(np.max(np.abs(pa["sharpness"] - pb["sharpness"]) / np.maximum(1e-3, np.abs(pa["sharpness"]))))
     return out
+
+
+def reference_summary(r1, r2, seed, sample=32):
+    """What is kept of two reference ExtractSift runs on one input (both in canonical order): the counts, sha256 of
+    the fields that must match bit for bit, every orientation, the run-to-run noise of orientations and descriptors,
+    the rows whose descriptor is not finite, and the descriptors of a seeded sample of rows (sample=None: all rows)."""
+    import hashlib
+    assert len(r1) == len(r2), (len(r1), len(r2))
+    out = {"count1": np.int32(len(r1)), "count2": np.int32(len(r2))}
+    for f in ("xpos", "ypos", "scale", "sharpness", "edgeness", "subsampling"):
+        out[f + "_sha"] = hashlib.sha256(np.ascontiguousarray(r1[f]).tobytes()).hexdigest()
+    do = np.abs(r1["orientation"] - r2["orientation"]) % 360.0
+    fin1 = np.isfinite(r1["data"]).all(axis=1)
+    fin = fin1 & np.isfinite(r2["data"]).all(axis=1)
+    dn = np.abs(r1["data"][fin] - r2["data"][fin]).max(axis=1)
+    n = len(r1) if sample is None else min(sample, len(r1))
+    rows = np.sort(np.random.default_rng(seed).choice(len(r1), n, replace=False)).astype(np.int32)
+    out.update(orientation=r1["orientation"].copy(), ori_noise=float(np.minimum(do, 360.0 - do).max()),
+               desc_noise=float(dn.max()), desc_bad_noise=np.int32((dn > 2e-5).sum()),
+               nonfinite=np.nonzero(~fin1)[0].astype(np.int32), rows=rows, data=r1["data"][rows].copy())
+    return out

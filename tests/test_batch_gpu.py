@@ -1,6 +1,8 @@
 """GPU tests of the batched TMA pipeline (round 2): identical to the round-1 per-image kernels (which are pinned to the
 reference), batches equal single images, the reference's cap of 32 extrema per block."""
 import ctypes
+import hashlib
+import os
 
 import numpy as np
 import pytest
@@ -12,6 +14,11 @@ from cudasift_b200.synth import synth_image
 pytestmark = pytest.mark.gpu
 
 FIELDS = ("xpos", "ypos", "scale", "sharpness", "edgeness", "orientation", "subsampling", "data")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+
+
+def sha(a):
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
 
 
 def canon(p):
@@ -164,15 +171,19 @@ def test_extrema_cap_mechanism_vs_oracle(cs):
     assert abs(len(a) - len(want)) <= 0.003 * len(want) + 2
 
 
-def test_dense_input_vs_reference(cs, reflib):
-    """Dense, low-threshold input against the reference itself: equal counts and positions (the cap included)."""
-    if reflib is None:
-        pytest.skip("oracle/_ref/libcudasift_ref.so not present")
+def dense_cases():
+    """Dense, low-threshold inputs and their thresholds: clipped noise, and a synthetic image."""
     rng = np.random.default_rng(5)
     noise = np.clip(128 + 60 * rng.standard_normal((480, 640)), 1, 254).astype(np.float32)
-    for arr, th in ((noise, 0.5), (synth_image(640, 480, seed=12), 0.1)):
-        ref = canon(reflib.extract(arr, thresh=th))
+    return ((noise, 0.5), (synth_image(640, 480, seed=12), 0.1))
+
+
+def test_dense_input_vs_reference(cs):
+    """Dense, low-threshold input against the reference itself (its results are stored in
+    tests/golden/reference_checks.npz): equal counts and positions (the cap included)."""
+    g = np.load(os.path.join(GOLDEN, "reference_checks.npz"))
+    for k, (arr, th) in enumerate(dense_cases()):
         got = canon(cs.extract_host(arr, thresh=th))
-        assert len(ref) == len(got) > 3000, (len(ref), len(got))
+        assert int(g["dense%d_count" % k]) == len(got) > 3000, (int(g["dense%d_count" % k]), len(got))
         for f in ("xpos", "ypos", "scale", "sharpness", "edgeness", "subsampling"):
-            assert np.array_equal(ref[f], got[f]), f
+            assert sha(got[f]) == str(g["dense%d_%s_sha" % (k, f)]), f

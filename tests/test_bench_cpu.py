@@ -51,7 +51,8 @@ def _load_bench(monkeypatch):
 
 
 def _args(impl):
-    return types.SimpleNamespace(gpus=1, steps=20, warmup=5, impl=impl, batch=32, rounds=0, streams=2, distinct=8, no_cpu=True)
+    return types.SimpleNamespace(gpus=1, steps=20, warmup=5, impl=impl, batch=32, rounds=0, streams=2, distinct=8, no_cpu=True,
+                                 dump_outputs=None)
 
 
 def test_both_arms_count_the_same_work(monkeypatch):
@@ -116,3 +117,40 @@ def test_both_arms_count_the_same_work(monkeypatch):
     assert prod["config"] == ref["config"]                                   # what the driver compares (same_config)
     assert prod["e2e"]["images"] >= 512 and prod["e2e"]["h2d_bytes_per_step"] == 384 * bench.W * bench.H * 4
     assert prod["gpu_launches"] == 20 * 12 * 2 * 6
+
+
+def test_dump_outputs_layout_and_cap(monkeypatch, tmp_path):
+    """--dump-outputs: float arrays only, images in order, each image's keypoints in canonical order whatever order the
+    device wrote them in, and a fixed seeded sample of rows (named in rows.npy) when the whole would exceed the cap."""
+    bench = _load_bench(monkeypatch)
+    from cudasift_b200.records import SIFT_DTYPE
+    rng = np.random.default_rng(1)
+    imgs = []
+    for n in (5, 0, 7):
+        p = np.zeros(n, SIFT_DTYPE)
+        for f in bench.DUMP_FIELDS:
+            p[f] = rng.random(n)
+        p["data"] = rng.random((n, 128))
+        imgs.append(p)
+
+    def load(d):
+        return {f[:-4]: np.load(os.path.join(d, f)) for f in sorted(os.listdir(d))}
+    bench.dump_outputs(str(tmp_path / "a"), imgs)
+    bench.dump_outputs(str(tmp_path / "b"), [p[::-1] for p in imgs])          # another arrival order
+    a, b = load(tmp_path / "a"), load(tmp_path / "b")
+    assert sorted(a) == ["counts", "descriptors", "keypoints"]
+    for k in a:
+        assert a[k].dtype in (np.float32, np.float64) and np.array_equal(a[k], b[k]), k
+    assert a["counts"].tolist() == [5, 0, 7] and a["keypoints"].shape == (12, 7) and a["descriptors"].shape == (12, 128)
+    first = np.sort(imgs[0], order=["subsampling", "ypos", "xpos", "scale", "orientation"])
+    assert np.array_equal(a["keypoints"][:5, 0], first["xpos"]) and np.array_equal(a["descriptors"][:5], first["data"])
+    row_bytes = 4 * (7 + 128)
+    cap = 3 * 8 + 4 * 128 + 6 * (row_bytes + 8)                                # room for 6 of the 12 rows
+    monkeypatch.setattr(bench, "DUMP_MAX_BYTES", cap)
+    bench.dump_outputs(str(tmp_path / "c"), imgs)
+    bench.dump_outputs(str(tmp_path / "d"), imgs)
+    c, d = load(tmp_path / "c"), load(tmp_path / "d")
+    rows = c["rows"].astype(int)
+    assert len(rows) == 6 and np.all(np.diff(rows) > 0) and np.array_equal(c["rows"], d["rows"])
+    assert np.array_equal(c["keypoints"], a["keypoints"][rows]) and np.array_equal(c["descriptors"], a["descriptors"][rows])
+    assert sum(v.nbytes for v in c.values()) <= cap

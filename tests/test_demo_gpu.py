@@ -10,7 +10,6 @@ import pytest
 from cudasift_b200 import build as _build
 from cudasift_b200.synth import synth_image
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def _write_pgm(path, img):
@@ -62,10 +61,12 @@ def test_demo_png_input_and_reference_drawing(cs, tmp_path):
     PrintMatchData (mainSift.cpp:150-200).  The demo decodes PNG itself (zlib) and --style reference draws the same
     primitives; feature counts must equal the ctypes API on the identically converted grey image."""
     cv2 = pytest.importorskip("cv2")
-    p1 = os.path.join(ROOT, "oracle", "_ref", "data", "img1.png")
-    p2 = os.path.join(ROOT, "oracle", "_ref", "data", "img2.png")
-    if not (os.path.exists(p1) and os.path.exists(p2)):
-        pytest.skip("oracle/_ref/data/img1.png, img2.png did not travel (built only where /root/reference exists)")
+    # a colour pair in the demo photographs' size (1920x1080 RGB), the second shifted: three different channels, so
+    # that the colour-to-grey conversion matters
+    base = [np.clip(synth_image(1920, 1080, seed=s), 0, 255).astype(np.uint8) for s in (61, 62)]
+    bgr = np.stack([base[0], np.roll(base[0], 3, axis=1), base[1]], axis=2)
+    p1, p2 = str(tmp_path / "img1.png"), str(tmp_path / "img2.png")
+    assert cv2.imwrite(p1, bgr) and cv2.imwrite(p2, np.roll(bgr, (9, -13), axis=(0, 1)))
     demo = _build.build_demo()
     out = str(tmp_path / "drawn.pgm")
     (n1, n2), (fit, matches), log = _run_demo(demo, [p1, p2, "--thresh", "2.0", "--repeat", "1", "--out", out, "--style", "reference"])

@@ -1,8 +1,6 @@
 """FindHomography (matching.cu:1000-1087), the consumer of MatchSiftData's output (SURVEY 8f-1).
 CPU: the oracle recovers a planted homography.  GPU: product == oracle under the same srand()
-seed, and == the reference library when it travelled."""
-import ctypes
-
+seed, and == the stored result of the reference library."""
 import numpy as np
 import pytest
 
@@ -56,24 +54,16 @@ def test_find_homography_equals_oracle(cs):
 
 
 @pytest.mark.gpu
-def test_find_homography_vs_reference(cs, reflib):
-    if reflib is None:
-        pytest.skip("oracle/_ref/libcudasift_ref.so not present")
-    import reflib as rl
+def test_find_homography_vs_reference(cs):
+    """Against the reference's FindHomography after srand(11) on the same points (tests/golden/reference_checks.npz)."""
+    import os
+    g = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_checks.npz"))
+    Hr, nr = g["homography_H"], int(g["homography_numfit"])
     p, _ = planted(n=1600, seed=9)            # multiple of 16: the reference reads no padding entries
-    f = reflib.L._Z14FindHomographyR8SiftDataPfPiifff
-    f.restype = ctypes.c_double
-    f.argtypes = [ctypes.POINTER(rl.CSiftData), ctypes.c_void_p, ctypes.POINTER(ctypes.c_int), ctypes.c_int,
-                  ctypes.c_float, ctypes.c_float, ctypes.c_float]
     sd = cs.InitSiftData(cs.SiftData(), 2048, False, True)
     sd._buf.upload(p); sd.numPts = len(p)
-    rsd = rl.CSiftData(len(p), 2048, None, sd.d_data)
-    Hr = np.zeros(9, np.float32); nr = ctypes.c_int(0)
-    ctypes.CDLL(None).srand(11)
-    with rl.quiet_stdout():
-        f(ctypes.byref(rsd), Hr.ctypes.data, ctypes.byref(nr), 2000, 0.85, 0.95, 4.0)
     Hg, ng, _ = cs.FindHomography(sd, 2000, 0.85, 0.95, 4.0, seed=11)
-    assert abs(ng - nr.value) <= max(2, 0.005 * nr.value), (ng, nr.value)
+    assert abs(ng - nr) <= max(2, 0.005 * nr), (ng, nr)
     assert np.allclose(Hg.ravel()[:8], Hr[:8], rtol=2e-3, atol=1e-5), (Hg, Hr)
 
 
